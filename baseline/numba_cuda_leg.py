@@ -5,9 +5,8 @@ Numba-CUDA path on 1 GPU ... in the same run").
 
 Runs in its OWN process (bench.py spawns it before it touches CUDA itself) so that numba's CUDA context, its JIT
 cache and the reference's import-time GPU query never share a process with the engine.  The reference is used
-UNMODIFIED through its public API, imported from where it lies: /root/reference (build container) or the
-git-ignored scratch copy baseline/_ref/ that travels with the snapshot to the GPU box; nothing of it is copied into
-the repository.  One shim: ``np.float = float`` (mppi_numba/mppi.py:32-33 uses the alias numpy removed).
+UNMODIFIED through its public API, imported from a checkout placed at baseline/_ref/ (git-ignored); nothing of it
+is part of the repository.  One shim: ``np.float = float`` (mppi_numba/mppi.py:32-33 uses the alias numpy removed).
 
     python baseline/numba_cuda_leg.py c5 [c3 c2 c4]      ->  ONE JSON line on stdout
 
@@ -29,10 +28,8 @@ ROOT = os.path.dirname(HERE)
 
 
 def locate():
-    for cand in ("/root/reference", os.path.join(HERE, "_ref")):
-        if os.path.isdir(os.path.join(cand, "mppi_numba")):
-            return cand
-    return None
+    cand = os.path.join(HERE, "_ref")
+    return cand if os.path.isdir(os.path.join(cand, "mppi_numba")) else None
 
 
 def main():
@@ -43,7 +40,7 @@ def main():
         os.write(real_stdout, (json.dumps(obj) + "\n").encode())
     ref_root = locate()
     if ref_root is None:
-        return emit({"unavailable": "reference package not found (/root/reference, baseline/_ref)"})
+        return emit({"unavailable": "reference package not found (baseline/_ref)"})
     try:
         import numpy as np
         np.float = float

@@ -28,6 +28,11 @@ own peer-memory kernels over NVLink (B200MPPI_EXCHANGE=nccl: by two NCCL collect
 `cpu_baseline`: the numpy oracle (oracle/mppi_ref.py) on a bounded N-slice, on this box's host cores.
 --impl reference: times that CPU path alone (the reference has no CPU implementation of its own; its GPU path is
 the numba_cuda_baseline leg above).
+--dump-outputs DIR: after the device-timed steps, what the last of them returned is written as DIR/u.npy (the T x 2
+           control sequence) and DIR/costs.npy (the N CVaR costs, all ranks' slices in order), float32.  The steps
+           before the timed ones are fixed by the arguments (see run_b200), so two builds can be compared output for
+           output.
+The benchmark runs from the tree build() left and writes nothing into it (it may be read-only).
 """
 import argparse
 import json
@@ -39,6 +44,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True          # no __pycache__ in the tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -254,7 +260,8 @@ def numba_cuda_leg(names, timeout_s=900):
     """The reference's Numba-CUDA path on this GPU, in a subprocess (its own CUDA context): baseline/numba_cuda_leg.py."""
     cmd = [sys.executable, os.path.join(ROOT, "baseline", "numba_cuda_leg.py")] + list(names)
     try:
-        r = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout_s, cwd=ROOT)
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout_s, cwd=ROOT,
+                           env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
         lines = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
         if not lines:
             return {"unavailable": "no output (rc %d): %s" % (r.returncode, r.stderr[-300:])}
@@ -444,9 +451,7 @@ def run_b200(args, sc):
     import torch
     if world != args.gpus:
         raise SystemExit("--gpus %d but WORLD_SIZE=%d: launch with torch.distributed.run" % (args.gpus, world))
-    import __graft_entry__
-    __graft_entry__.build()
-    import mppi_numba_b200 as E
+    import mppi_numba_b200 as E           # the library build() compiled (importing fails loudly without it)
     torch.cuda.set_device(local)
     pg = None
     if world > 1:
@@ -505,8 +510,13 @@ def run_b200(args, sc):
     # multi-rank run contains exchanges, so the NUMBER of extra solves must be the same on every rank:
     # agree on it (max over ranks) instead of looping on each rank's own wall clock.
     n_settle = int(max_over_ranks(float(min(5000, int(0.5 / per_solve) + 1))))
+    # that number depends on the wall clock: the settle solves start from a checkpoint (warm start + RNG streams)
+    # that is restored after them, so the timed steps are always solves warmup+1 .. warmup+K of the seeded planner
+    checkpoint = pl.get_state()
     for _ in range(n_settle):
         pl.solve()
+    barrier()
+    pl.set_state(checkpoint)
     barrier()
     clocks.lines.clear()
     l0 = pl.launch_count()          # includes the TDM kernels launched inside solve()
@@ -519,6 +529,14 @@ def run_b200(args, sc):
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     launches = pl.launch_count() - l0      # kernels launched in the timed region
+    if args.dump_outputs:
+        costs = pl.costs_d.copy_to_host()
+        if world > 1:
+            import torch.distributed as dist
+            parts = [None] * world
+            dist.all_gather_object(parts, costs)
+            costs = np.concatenate(parts)
+        dump = {"u": u, "costs": costs}
     # very short timed region: extend the load for the clock sampler only (same count on every rank)
     if max_over_ranks(1.0 if len(clocks.lines) < 3 else 0.0) > 0.0:
         for _ in range(int(min(5000, int(0.4 / (ms * 1e-3)) + 1))):
@@ -623,7 +641,7 @@ def run_b200(args, sc):
         res = {}
         for name in others:
             try:
-                res[name] = time_small_workload(E, torch, name, local, max(args.steps, 20), args.warmup)
+                res[name] = time_small_workload(E, torch, name, local, args.steps, args.warmup)
                 w = (numba or {}).get("workloads", {}).get(name)
                 if w:
                     res[name]["numba_cuda_ms_per_solve"] = w["ms_per_solve"]
@@ -632,6 +650,10 @@ def run_b200(args, sc):
                 res[name] = {"error": repr(e)}
         out["others"] = res
     if rank == 0:
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
         _emit(json.dumps(out))
     if world > 1:
         import torch.distributed as dist
@@ -661,7 +683,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-numba", action="store_true", help="skip the reference's Numba-CUDA leg (N = 1)")
     ap.add_argument("--no-others", action="store_true", help="skip the other BASELINE configs (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write u and the CVaR costs of the last timed solve to DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     sc = build_scenario(args.workload)
     if args.impl == "reference":
