@@ -231,8 +231,201 @@ def make_state_rollout_golden(Config, TDM_Numba, MPPI_Numba):
     np.savez_compressed(os.path.join(OUT, "ref_state_rollout.npz"), **out)
 
 
+# Planner parameter points away from the defaults.  At the defaults (lambda 1, traction bounds [0, 1], vrange [0, 3],
+# a symmetric wrange, dist_weight 1, ...) several wrong formulas give the right numbers; each value below breaks one
+# such tie: lambda != 1, lo != 0 and a traction range != 1 (bounds), |v| != v (vrange[0] < 0 at P1), vrange[0] > 0
+# (P2), w_lo != -w_hi, dist_weight != 1, u_std whose squares are not exact in float32, non-default penalties (an
+# obstacle penalty of 0 at P2), non-dyadic resolutions.  P1 also has mask bytes above 1 (the general penalty
+# variant) and one sampled map with bytes over the whole int8 range.
+PARAM_POINTS = dict(
+    p1=dict(lin_bounds=[-0.25, 1.6], ang_bounds=[0.2, 0.85], vrange=[-1.5, 2.2], wrange=[-0.9, 2.1], u_std=[0.7, 1.9],
+            lam=0.37, dt=0.07, dist_weight=2.5, goal_tol=0.8, v_post=0.35, obs_cost=3.5e3, unk_cost=17.0, res=0.3,
+            x0=[2.7, 5.9, 0.4], xgoal_near=[3.4, 6.3], xgoal_far=[30.0, 30.0], u_lo=[-1.0, -0.5], u_hi=[2.0, 1.5],
+            wild_map=True, masks_general=True, obs_cells=[(12, 11, 3), (14, 13, 1)], unk_cells=[(13, 13, 2)]),
+    p2=dict(lin_bounds=[0.1, 0.6], ang_bounds=[-1.0, 1.0], vrange=[0.5, 4.0], wrange=[-2.5, 0.4], u_std=[3.3, 0.45],
+            lam=4.2, dt=0.25, dist_weight=0.3, goal_tol=0.05, v_post=2.0, obs_cost=0.0, unk_cost=250.0, res=0.55,
+            x0=[5.1, 8.4, 2.2], xgoal_near=[4.2, 9.2], xgoal_far=[-30.0, 40.0], u_lo=[0.5, -2.0], u_hi=[3.0, 0.3],
+            wild_map=False, masks_general=False, obs_cells=[(12, 9, 1)], unk_cells=[(13, 9, 1), (15, 8, 1)]),
+)
+
+# the whole-solve sequence at P1.  The reference's PMF setter requires bin values and bounds that start at 0
+# (terrain.py:403-404), so the solve keeps lo = 0 with P1's traction ranges (lo != 0 is covered kernel by kernel above).
+# Bin values whose quantised bytes 100 * v / hi lie far from an integer: the simulator's float32 typing and the
+# compiled float64 typing truncate them to the same byte.
+PARAMS_SOLVE = dict(lin_bounds=[0.0, 1.6], ang_bounds=[0.0, 0.85], lin_bin_values=[0.0, 0.3, 0.9, 1.4, 1.55],
+                    ang_bin_values=[0.0, 0.22, 0.4, 0.6, 0.84], B=5, H=24,
+                    W=24, N=100, M=4, T_s=0.6, seed=3, thread_dim=[4, 4], max_speed_padding=5.0, det_alpha=0.4,
+                    x0=[3.6, 3.5, 0.9], xgoal=[5.2, 4.6], x0_next=[3.7, 3.55, 0.95], cvar_alpha=0.7, alpha_dyn=0.8)
+
+
+def params_point_inputs(name):
+    """The small rollout inputs of ref_rollout.npz (M 6, 26 x 24 maps, N 24, T 12), noise scaled by the point's u_std."""
+    P = PARAM_POINTS[name]
+    f32 = np.float32
+    g = np.load(os.path.join(OUT, "ref_rollout.npz"))
+    rng = np.random.default_rng(dict(p1=101, p2=202)[name])
+    lin, ang = g["lin"].copy(), g["ang"].copy()
+    obs, unk = g["obs"].copy(), g["unk"].copy()
+    M, R, C = lin.shape
+    Hp, Wp = obs.shape
+    if P["wild_map"]:                                    # bytes outside 0..100, negative ones included
+        lin[2] = rng.integers(-128, 128, (R, C)).astype(np.int8)
+        ang[4] = rng.integers(-128, 128, (R, C)).astype(np.int8)
+    if P["masks_general"]:                               # mask bytes > 1: the general penalty arithmetic
+        obs = (obs * rng.integers(1, 4, obs.shape)).astype(np.int8)
+        unk = (unk * rng.integers(1, 3, unk.shape)).astype(np.int8)
+        assert obs.max() > 1 and unk.max() > 1
+    for r, c, v in P["obs_cells"]:                       # cells on the rollouts' paths (the robot moves a few cells)
+        obs[r, c] = v
+    for r, c, v in P["unk_cells"]:
+        unk[r, c] = v
+    res = f32(P["res"])
+    xlim = np.array([-1.0, -1.0 + Wp * res], dtype=f32)
+    ylim = np.array([2.0, 2.0 + Hp * res], dtype=f32)
+    N, T = g["noise"].shape[:2]
+    noise = (rng.standard_normal((N, T, 2)) * np.array(P["u_std"])).astype(f32)
+    u_cur = np.stack([rng.uniform(P["u_lo"][0], P["u_hi"][0], T), rng.uniform(P["u_lo"][1], P["u_hi"][1], T)], 1).astype(f32)
+    d = dict(lin=lin, ang=ang, obs=obs, unk=unk, risk=g["risk"], res=res, xlim=xlim, ylim=ylim, noise=noise, u_cur=u_cur,
+             x0=np.array(P["x0"], f32), xgoal_near=np.array(P["xgoal_near"], f32), xgoal_far=np.array(P["xgoal_far"], f32))
+    for k in ("lin_bounds", "ang_bounds", "vrange", "wrange", "u_std"):
+        d[k] = np.array(P[k], dtype=np.float64)
+    for k in ("lam", "dt", "dist_weight", "goal_tol", "v_post", "obs_cost", "unk_cost"):
+        d[k] = np.float64(P[k])
+    return d
+
+
+def make_params_golden(Config, TDM_Numba, MPPI_Numba, cuda):
+    """Reference kernels at the PARAM_POINTS (tests/test_params_emulated_cpu.py, tests/test_gpu_params.py): per-(n,m)
+    stochastic costs, CVaR at alpha 0.5 / 0.9, the deterministic and speed-map kernels, the update kernel; and at P1 a
+    whole solve() -> shift_and_update() -> solve() through the public API in the three modes."""
+    from oracle import mppi_ref as MR
+    f32 = np.float32
+    dev = cuda.to_device
+    out = {}
+    for name in sorted(PARAM_POINTS):
+        d = params_point_inputs(name)
+        N, T = d["noise"].shape[:2]
+        M = d["lin"].shape[0]
+        Hp, Wp = d["obs"].shape
+
+        def arr(k):
+            return dev(np.asarray(d[k], f32))
+
+        def scal(k):
+            return f32(d[k])
+
+        for gname in ("near", "far"):
+            goal = d["xgoal_" + gname]
+            # every lookup of every rollout stays inside the mask arrays (the reference does not bound its indices)
+            _, st = MR.rollout_costs(MR.MODE_STOCHASTIC, d["lin"], d["ang"], d["lin_bounds"], d["ang_bounds"], d["obs"],
+                                     d["unk"], d["res"], d["xlim"], d["ylim"], d["vrange"], d["wrange"], goal, d["v_post"],
+                                     d["obs_cost"], d["unk_cost"], d["goal_tol"], d["lam"], d["u_std"], d["x0"], d["dt"],
+                                     d["dist_weight"], d["noise"], d["u_cur"], return_states=True)
+            xi = np.floor((st[..., 0].astype(np.float64) - d["xlim"][0]) / d["res"])
+            yi = np.floor((st[..., 1].astype(np.float64) - d["ylim"][0]) / d["res"])
+            assert xi.min() >= 1 and yi.min() >= 1 and xi.max() < Wp - 1 and yi.max() < Hp - 1, (name, gname)
+
+            def launch_sto(alpha, gl, ga, block):
+                costs_d = cuda.device_array((N,), dtype=f32)
+                MPPI_Numba.rollout_numba[N, block, 0, 4 * block](
+                    dev(gl), dev(ga), arr("lin_bounds"), arr("ang_bounds"), dev(d["obs"]), dev(d["unk"]), d["res"],
+                    dev(d["xlim"]), dev(d["ylim"]), arr("vrange"), arr("wrange"), dev(goal), scal("v_post"),
+                    scal("obs_cost"), scal("unk_cost"), scal("goal_tol"), scal("lam"), arr("u_std"), f32(alpha),
+                    dev(d["x0"]), scal("dt"), float(d["dist_weight"]), dev(d["noise"]), dev(d["u_cur"]), costs_d)
+                return costs_d.copy_to_host()
+
+            def launch_det(speed_map):
+                costs_d = cuda.device_array((N,), dtype=f32)
+                args = [dev(d["lin"][:1]), dev(d["ang"][:1])] + ([dev(d["risk"])] if speed_map else [])
+                args += [arr("lin_bounds"), arr("ang_bounds"), dev(d["obs"]), dev(d["unk"]), d["res"], dev(d["xlim"]),
+                         dev(d["ylim"]), arr("vrange"), arr("wrange"), dev(goal), scal("v_post"), scal("obs_cost"),
+                         scal("unk_cost"), scal("goal_tol"), scal("lam"), arr("u_std"), dev(d["x0"]), scal("dt"),
+                         float(d["dist_weight"]), dev(d["noise"]), dev(d["u_cur"]), costs_d]
+                k = MPPI_Numba.rollout_det_dyn_w_speed_map_numba if speed_map else MPPI_Numba.rollout_det_dyn_numba
+                k[N, 1](*args)
+                return costs_d.copy_to_host()
+
+            d["sto_cnm_" + gname] = np.stack([launch_sto(1.0, d["lin"][m:m + 1], d["ang"][m:m + 1], 1)
+                                              for m in range(M)], 1)
+            for alpha in (0.5, 0.9):
+                d["sto_cvar%02d_%s" % (int(alpha * 10), gname)] = launch_sto(alpha, d["lin"], d["ang"], M)
+            d["det_" + gname] = launch_det(False)
+            d["spd_" + gname] = launch_det(True)
+            print("params", name, gname, "done")
+
+        # update: 320 control sequences, three slabs of 32 with penalty-sized costs (weights underflow to 0)
+        rng = np.random.default_rng(dict(p1=103, p2=203)[name])
+        Nu, Tu = 320, 9
+        costs = rng.uniform(20, 30, Nu).astype(f32)
+        costs[64:160] += rng.uniform(0.9e5, 1.1e5, 96).astype(f32)
+        costs[250:290] += f32(d["unk_cost"]) * rng.integers(1, 4, 40).astype(f32)
+        noise_u = (rng.standard_normal((Nu, Tu, 2)) * d["u_std"]).astype(f32)
+        P = PARAM_POINTS[name]
+        u0 = np.stack([rng.uniform(P["u_lo"][0], P["u_hi"][0], Tu), rng.uniform(P["u_lo"][1], P["u_hi"][1], Tu)], 1)
+        u0 = u0.astype(f32)
+        c_d, w_d, u_d = dev(costs.copy()), cuda.device_array((Nu,), dtype=f32), dev(u0.copy())
+        MPPI_Numba.update_useq_numba[1, 1](scal("lam"), c_d, dev(noise_u), w_d, arr("vrange"), arr("wrange"), u_d)
+        d.update(upd_costs=costs, upd_noise=noise_u, upd_u0=u0, upd_u=u_d.copy_to_host(), upd_w=w_d.copy_to_host())
+        out.update({name + "_" + k: v for k, v in d.items()})
+        print("params", name, "update done")
+
+    # ---- whole solve at P1 through the public API, three modes
+    S, P = PARAMS_SOLVE, PARAM_POINTS["p1"]
+    rng = np.random.default_rng(19)
+    B, H, W = S["B"], S["H"], S["W"]
+    pmf_l = random_pmf(rng, B, H, W, zero_frac=0.2)
+    pmf_a = random_pmf(rng, B, H, W, zero_frac=0.2)
+    obstacle = (rng.random((H, W)) < 0.05).astype(np.int8)
+    unknown = (rng.random((H, W)) < 0.05).astype(np.int8)
+    res = P["res"]
+    mmd = (H + 2 * 2, W + 2 * 2)
+    out.update(solve_pmf_lin=pmf_l, solve_pmf_ang=pmf_a, solve_obstacle=obstacle, solve_unknown=unknown, solve_res=res,
+               solve_max_map_dim=np.array(mmd), **{"solve_" + k: np.asarray(v) for k, v in S.items()})
+    params = dict(dt=P["dt"], x0=np.array(S["x0"]), xgoal=np.array(S["xgoal"]), goal_tolerance=P["goal_tol"],
+                  v_post_rollout=P["v_post"], cvar_alpha=S["cvar_alpha"], alpha_dyn=S["alpha_dyn"],
+                  dist_weight=P["dist_weight"], lambda_weight=P["lam"], num_opt=1, u_std=np.array(P["u_std"]),
+                  vrange=np.array(P["vrange"]), wrange=np.array(P["wrange"]), obs_penalty=P["obs_cost"],
+                  unknown_penalty=P["unk_cost"])
+    for mode, flags in (("tdm", dict(use_tdm=True)), ("det", dict(use_det_dynamics=True)),
+                        ("spd", dict(use_nom_dynamics_with_speed_map=True))):
+        cfg = _quiet(Config, T=S["T_s"], dt=P["dt"], num_grid_samples=S["M"], num_control_rollouts=S["N"], seed=S["seed"],
+                     max_map_dim=mmd, tdm_sample_thread_dim=tuple(S["thread_dim"]),
+                     max_speed_padding=S["max_speed_padding"], num_vis_state_rollouts=5, **flags)
+        lt, at = _quiet(TDM_Numba, cfg), _quiet(TDM_Numba, cfg)
+        for t_, pmf, which in ((lt, pmf_l, "lin"), (at, pmf_a, "ang")):
+            dd = dict(res=res, xlimits=np.array([0.0, W * res]), ylimits=np.array([0.0, H * res]),
+                      bin_values=np.array(S[which + "_bin_values"]), bin_values_bounds=np.array(S[which + "_bounds"]),
+                      det_dynamics_cvar_alpha=S["det_alpha"])
+            _quiet(t_.set_TDM_from_PMF_grid, pmf, dd, obstacle, unknown)
+            t_.sample_grid_batch_d.copy_to_device(np.zeros(t_.sample_grid_batch_d.shape, dtype=np.int8))
+        assert cfg.num_steps == 8, cfg.num_steps
+        pl = _quiet(MPPI_Numba, cfg)
+        pl.setup(dict(params, x0=params["x0"].copy()), lt, at)
+        orig = MPPI_Numba.update_useq_numba
+
+        class _One:                                  # SURVEY 9-R1: the update kernel is racy with 32 threads
+            def __getitem__(self, cfg_):
+                return orig[1, 1]
+        pl.update_useq_numba = _One()
+        u1 = _quiet(pl.solve).copy()
+        out["solve_%s_u1" % mode] = u1
+        out["solve_%s_noise1" % mode] = pl.noise_samples_d.copy_to_host().copy()
+        out["solve_%s_lin_grid1" % mode] = lt.sample_grid_batch_d.copy_to_host().copy()
+        out["solve_%s_ang_grid1" % mode] = at.sample_grid_batch_d.copy_to_host().copy()
+        out["solve_%s_states1" % mode] = _quiet(pl.get_state_rollout).copy()
+        pl.shift_and_update(np.array(S["x0_next"]), u1, num_shifts=1)
+        out["solve_%s_u2" % mode] = _quiet(pl.solve).copy()
+        out["solve_%s_weights2" % mode] = pl.weights_d.copy_to_host().copy()
+        print("params solve", mode, "done")
+    np.savez_compressed(os.path.join(OUT, "ref_params.npz"), **out)
+
+
 def main():
     from oracle.ref_loader import load_reference
+    if "--only-params" in sys.argv:
+        Config, TDM_Numba, MPPI_Numba, cuda = load_reference()
+        make_params_golden(Config, TDM_Numba, MPPI_Numba, cuda)
+        return
     if "--only-state-rollout" in sys.argv:
         Config, TDM_Numba, MPPI_Numba, cuda = load_reference()
         make_state_rollout_golden(Config, TDM_Numba, MPPI_Numba)
@@ -436,6 +629,7 @@ def main():
         print("solve", mode, "done")
     np.savez_compressed(os.path.join(OUT, "ref_solve.npz"), **solve)
     make_state_rollout_golden(Config, TDM_Numba, MPPI_Numba)     # get_state_rollout after the first solve
+    make_params_golden(Config, TDM_Numba, MPPI_Numba, cuda)      # non-default planner parameters (reuses section 3)
 
 
 if __name__ == "__main__":

@@ -19,8 +19,11 @@ def random_pmf(rng, B, H, W):
 
 def make_scenario(mode, N, M, T, H, W, res, B, seed=1, near_goal=False, warm_start=False,
                   det_alpha=1.0, cvar_alpha=0.5, pad_speed=5.0, thread_dim=(16, 16), bin_values=None,
-                  mask_p=0.01):
-    dt = 0.1
+                  mask_p=0.01, bin_bounds=(0.0, 1.0), dt=0.1, params=None):
+    """``bin_values`` / ``bin_bounds``: the traction bins and bounds of both maps (default: B values evenly over
+    [0, 1]); ``params``: entries that replace or extend the planner's params dict (``dt`` is set here, because the
+    horizon and the map padding depend on it)."""
+    overrides = dict(params or {})
     pad = int(np.ceil(pad_speed * dt / res))
     flags = dict(tdm=dict(use_tdm=True), det=dict(use_det_dynamics=True),
                  spd=dict(use_nom_dynamics_with_speed_map=True))[mode]
@@ -38,13 +41,14 @@ def make_scenario(mode, N, M, T, H, W, res, B, seed=1, near_goal=False, warm_sta
     obstacle[int(x0[1] / res), int(x0[0] / res)] = 0
     xgoal = x0[:2] + (np.array([1.2, 1.2]) * min(1.0, L / 20) if near_goal else 0.42 * L * np.ones(2))
     if bin_values is None:
-        bin_values = np.linspace(0, 1, B)
+        bin_values = np.linspace(bin_bounds[0], bin_bounds[1], B)
     tdm_dict = dict(res=res, xlimits=np.array([0.0, W * res]), ylimits=np.array([0.0, H * res]),
-                    bin_values=np.asarray(bin_values), bin_values_bounds=np.array([0.0, 1.0]),
+                    bin_values=np.asarray(bin_values), bin_values_bounds=np.array(bin_bounds, dtype=float),
                     det_dynamics_cvar_alpha=det_alpha)
     params = dict(dt=dt, x0=x0, xgoal=xgoal, goal_tolerance=0.5, v_post_rollout=0.01, cvar_alpha=cvar_alpha,
                   alpha_dyn=1.0, dist_weight=1.0, lambda_weight=1.0, num_opt=1, u_std=np.array([2.0, 3.0]),
                   vrange=np.array([0.0, 3.0]), wrange=np.array([-np.pi, np.pi]))
+    params.update(overrides)
     sc = dict(mode=mode, cfg=cfg, pmf_lin=pmf_lin, pmf_ang=pmf_ang, obstacle=obstacle, unknown=unknown,
               tdm_dict=tdm_dict, params=params, N=N, M=M, T=T)
     if warm_start:
